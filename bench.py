@@ -19,12 +19,15 @@ purge / serialise -> K5 LZ4|Snappy + CRC32) of one batch of synthetic input SSTa
   verified         the output of the timed configuration — device-resident AND streamed through host buffers — compared byte for byte
                    (Data.db, Index.db, chunk offsets, Digest.crc32, counters) with the CPU oracle's output for the same inputs.
 --impl reference   the CPU oracle with all host threads on the same workload, same metric/unit (+ its scaling curve over threads).
+--dump-outputs DIR the output files of the last timed device-resident step as DIR/<name>.npy (see dump_outputs), so that two builds can be
+                   compared output for output: the inputs are seeded, identical from run to run for the same arguments.
 Input synthesis (synth/) never touches oracle/: the b200 arm compresses its inputs with the engine's own K5 kernels.
 """
 import argparse, ctypes as C, json, os, subprocess, sys, threading, time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: nothing is cached next to the sources
 NOW = 1700000000
 METRIC = "compaction MB/s (uncompressed in)"
 INT64_MIN, INT64_MAX = -(1 << 63), (1 << 63) - 1
@@ -277,6 +280,35 @@ def same_files(a, b):
         if x[3:] != y[3:]: return "file %d: digest/partitions/rows %s vs %s" % (k, x[3:], y[3:])
     return None
 
+DUMP_SAMPLES = {"data": 2 << 20, "index": 1 << 20, "chunk_offsets": 1 << 19}    # elements per job, split over its output files: < 64 MB in all
+
+def sample_positions(n, cap, seed):
+    """sorted positions of a stratified sample of cap of n elements, fixed by seed (every position when n <= cap)"""
+    import numpy as np
+    if n <= cap: return np.arange(n, dtype=np.int64)
+    stride = n // cap
+    return np.arange(cap, dtype=np.int64) * stride + np.random.default_rng(seed).integers(0, stride, cap)
+
+def dump_outputs(ob, res, ninputs):
+    """What a caller of b200c_compact receives, as float arrays. For output file k: out<k>_data, out<k>_index, out<k>_chunk_offsets hold the
+    Data.db bytes, Index.db bytes and chunk offsets at the positions in out<k>_<name>_pos (a fixed, seeded sample of large files). `files` has
+    one row per output: data_len, index_len, nchunks, data_length, digest (CRC32 of all of Data.db), CRC32 of all of Index.db, CRC32 of all
+    chunk offsets, partitions, rows. `counters`: bytes_read, bytes_in_range, bytes_written, total_source_rows, input_partitions, merged_row_counts."""
+    import numpy as np, torch, zlib
+    out, files = {}, []
+    for k in range(res.noutputs):
+        o = res.outputs[k]; d, ix, co = ob.bufs[k]
+        for j, (name, t, dt) in enumerate((("data", d[:o.data_len], np.float32), ("index", ix[:o.index_len], np.float32), ("chunk_offsets", co[:o.nchunks], np.float64))):
+            pos = sample_positions(t.numel(), DUMP_SAMPLES[name] // res.noutputs, seed=1000 * k + j)
+            out["out%d_%s" % (k, name)] = t[torch.from_numpy(pos).to(t.device)].cpu().numpy().astype(dt)
+            out["out%d_%s_pos" % (k, name)] = pos.astype(np.float64)
+        files.append([o.data_len, o.index_len, o.nchunks, o.data_length, o.digest, zlib.crc32(ix[:o.index_len].cpu().numpy()),
+                      zlib.crc32(co[:o.nchunks].cpu().numpy()), o.partitions, o.rows])
+    out["files"] = np.array(files, dtype=np.float64).reshape(-1, 9)
+    out["counters"] = np.array([res.bytes_read, res.bytes_in_range, res.bytes_written, res.total_source_rows, res.input_partitions] +
+                               [int(x) for x in res.merged_row_counts[:ninputs]], dtype=np.float64)
+    return out
+
 def estimate_max_ranges(u_in, threads, ranges, budget_s, per_thread_mbs=110.0):
     est = u_in / 1e6 / (per_thread_mbs * max(1, threads) * 0.7)
     if est <= budget_s: return 0, est
@@ -348,6 +380,7 @@ def run_b200(args, wl):
 
     for _ in range(args.warmup): step(True)
     dt, kms, stages, last, launches, clocks = timed(True, args.steps, ClockSampler(local))
+    dump = dump_outputs(do, last, len(tabs)) if args.dump_outputs else None     # before any later leg reuses the device buffers
     sum_outs = lambda res, f: sum(int(getattr(res.outputs[k], f)) for k in range(res.noutputs))
     u_out, c_out, i_out = int(last.bytes_written), sum_outs(last, "data_len"), sum_outs(last, "index_len")
     rows = int(last.total_source_rows); parts_in = int(last.input_partitions); in_range = int(last.bytes_in_range)
@@ -419,6 +452,12 @@ def run_b200(args, wl):
         cpu_leg_and_verify(args, wl, line, tabs, m_host, (cap_d, cap_i, cap_c, nout), ctx, L, do, ho, last, elast, build_manifest, dev_in)
     if rank == 0:
         emit(line)
+    if dump:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, ("rank%d_" % rank if world > 1 else "") + name + ".npy"), a)
+        log("wrote %d arrays (%.1f MB) to %s" % (len(dump), sum(a.nbytes for a in dump.values()) / 1e6, args.dump_outputs))
     ctx.close()
     if world > 1: dist.destroy_process_group()
 
@@ -559,7 +598,10 @@ def main():
     ap.add_argument("--cpu-budget-s", type=float, default=20.0, help="bound of one CPU-oracle compaction (cpu_baseline leg and reference arm)")
     ap.add_argument("--ref-threads", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU leg AND the verification (development)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write the last timed step's output files (a fixed sample of large ones) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1: ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference": ap.error("--dump-outputs writes what the b200 arm computed")
     wl = dict(WORKLOADS[args.workload]); wl["rpp"] = args.rows_per_partition
     if args.sstables or args.sstable_mib:
         if args.sstables: wl["sstables"] = args.sstables

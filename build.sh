@@ -1,5 +1,5 @@
 #!/bin/bash
-# Builds libb200compact.so (sm_100a only) in-tree, and the CPU oracle (test infrastructure).
+# Builds libb200compact.so (sm_100a only) in-tree, the CPU oracle (test infrastructure) and the input generator bench.py loads.
 set -e
 cd "$(dirname "$0")"
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
@@ -10,4 +10,5 @@ $NVCC -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompile
 mv -f $OUT.tmp $OUT          # atomically: a gpurun snapshot taken meanwhile sees the old or the new library, never half of one
 grep -E "error|warning" build_ptxas.log | grep -v "ptxas info" | head -20 || true
 make -C oracle -s
+make -C synth -s
 echo "built $OUT"

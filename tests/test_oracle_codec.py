@@ -1,6 +1,6 @@
-"""Pins the CPU oracle's codecs against (1) the reference's golden SSTables, (2) zlib, (3) the system liblz4.so.1.
+"""Pins the CPU oracle's codecs against (1) the reference's golden SSTables, (2) zlib, (3) liblz4 (stored digests, and liblz4.so.1 live).
 SURVEY §8c: compressed bytes are pinned only by the golden files; CRC32 by Data.db inline checksums + Digest.crc32."""
-import ctypes as C, os, random, struct, zlib, pytest
+import ctypes as C, hashlib, json, os, random, struct, zlib, pytest
 import oracle_lib as O
 from sstable_files import read_compression_info, split_chunks, find_tables
 
@@ -56,14 +56,20 @@ def _corpus(rng):
     return out
 
 def test_lz4_matches_system_liblz4():
+    # liblz4's output for the corpus is pinned by tests/golden/lz4/vectors.json (tests/golden/tools/make_lz4_vectors.py); where the library
+    # is installed, its live output is compared as well
+    want = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "lz4", "vectors.json")))["vectors"]
+    corpus = _corpus(random.Random(0xCA55))
+    assert len(want) == len(corpus)
     L = _liblz4()
-    if L is None: pytest.skip("no system liblz4")
-    rng = random.Random(0xCA55)
-    for s in _corpus(rng):
-        cap = O.lib().orc_lz4_compress_bound(len(s)); buf = C.create_string_buffer(cap + 1)
-        n = L.LZ4_compress_default(s, buf, len(s), cap)
-        assert O.lz4_compress(s) == buf.raw[:n], len(s)
-        assert O.lz4_decompress(buf.raw[:n], len(s)) == s
+    for s, w in zip(corpus, want):
+        c = O.lz4_compress(s)
+        assert (len(s), len(c), hashlib.sha256(c).hexdigest()) == (w["n"], w["compressed_len"], w["sha256"])
+        assert O.lz4_decompress(c, len(s)) == s
+        if L is not None:
+            cap = O.lib().orc_lz4_compress_bound(len(s)); buf = C.create_string_buffer(cap + 1)
+            n = L.LZ4_compress_default(s, buf, len(s), cap)
+            assert c == buf.raw[:n], len(s)
 
 def test_lz4_rejects_malformed():
     s = bytes(random.Random(1).getrandbits(8) for _ in range(500)) + b"x" * 500
