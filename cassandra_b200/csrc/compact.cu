@@ -799,6 +799,41 @@ __global__ void __launch_bounds__(ST_THREADS) k_partition_staged(const K4Args a,
     if (a.sg) stat_flush_warp(a.sg, acc);               // (no thread returns after the barrier wait: every lane gets here)
 }
 
+// ---- K4 statistics pass of one output file (multi-file output with the side band) ---------------------------------------------------
+// The file boundaries of a leveled compaction are known only after K5, so the per-cell / per-row reductions cannot come from the
+// serialisation pass. Per file, this runs the same process_partition() again over the written partitions jlo <= j < jhi in the
+// non-emitting (counting-sink) instantiation: nothing is written but the file's StatGlobal / TdropTable and ccount[j]. A kernel of
+// its own, so that the serialisation kernels keep their code. Every fan-in class takes the thread-per-partition mapping (64 cursors
+// per thread above 16; the warp kernels of those classes compute the same values). No lane returns early: the accumulators are folded
+// per warp (stat_flush_warp) before the StatGlobal atomics, one flush per warp instead of one per partition. A partition the kernel
+// refuses fails the call (the serialisation pass refused it first so far; a disagreement must not drop it from Statistics.db silently).
+template <int M_CAP, int NT, bool CX>
+__global__ void __launch_bounds__(NT) k_partition_stats(const K4Args a, uint64_t lo, uint64_t hi) {
+    extern __shared__ __align__(16) uint8_t s_raw[];
+    const int ncols_s = a.P->mcols <= K4_SMEM_COLS ? a.P->mcols : 0;
+    const int stride = M_CAP * SLOT_BYTES + ncols_s * (int)sizeof(MCell) + 8;
+    K4Cur* cur = (K4Cur*)(s_raw + (size_t)threadIdx.x * stride);
+    MCell merged_local[MAXCOLS];
+    MCell* merged = ncols_s ? (MCell*)(cur + M_CAP) : merged_local;
+    DT open_dt[M_CAP];
+    StatAcc acc; acc.init(a.P->now, a.td);
+    const uint64_t t = lo + (uint64_t)blockIdx.x * NT + threadIdx.x;
+    uint64_t j = 0; bool work = t < hi;
+    if (work) { j = a.list[t]; work = j >= a.jlo && j < a.jhi && a.dsize[j]; }
+    if (work) {
+        const uint64_t c0 = a.op_first[j]; const uint32_t m = (uint32_t)(a.op_first[j + 1] - c0);
+        PartOut out{0, 0, 0, 0, 0}; PartStats st{0, 0}; int e = 0;
+        if (m > (uint32_t)M_CAP) e = PERR_UNSUPPORTED;
+        else process_partition<false, K4Cur, XlateGlobal, M_CAP, CX>(*a.P, XlateGlobal(), a.contrib, c0, m, a.upos, a.pbase, a.kp, a.klen, a.tok, nullptr, ~0ull, 0, nullptr, 0, 0, 0, cur, open_dt, merged, out, st, e, &acc);
+        if (e) {
+            const uint64_t en = a.contrib[c0]; const int src = (int)((en >> 56) & 0x7F);
+            report_err(a.err, e == PERR_UNSUPPORTED ? 9 : 4, src, a.upos[a.pbase[src] + (en & 0xFFFFFFFFFFull)] - a.P->in[src].ubase);
+            acc.init(a.P->now, a.td);
+        } else a.ccount[j] = out.cells;
+    }
+    stat_flush_warp(a.sg, acc);                           // (block sizes are multiples of 32 and every lane gets here)
+}
+
 // upper bound of an output partition's size: the sum of its input partitions plus 25 % + 32 bytes (re-based deltas can lengthen
 // vints by a byte or two per field; a partition that still does not fit is caught by the overflow flag and re-emitted by mode 3)
 // icap[j]: bytes of promoted-index slot (0 when the partition cannot reach a second column-index block)
@@ -924,10 +959,10 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
     if (m->npurge_ranges < 0 || (m->npurge_ranges && (!m->purge_range_hi || !m->purge_range_max_ts))) { c->err = "purge table"; return B200C_EINVAL; }
     for (int k = 1; k < m->npurge_ranges; k++) if (m->purge_range_hi[k] <= m->purge_range_hi[k - 1]) { c->err = "purge_range_hi must ascend"; return B200C_EINVAL; }
     if (c->cancel.exchange(0)) { c->err = "cancelled"; return B200C_ECANCELLED; }        // stop requested before the task got here
-    // the rest of the sstable (Filter.db / Summary.db / Statistics.db side band / first+last key): single-output compactions
+    // the rest of the sstable (Filter.db / Summary.db / Statistics.db side band / first+last key), per output file; output 0 says which parts
     const b200c_output& o0 = res->outputs[0];
     const bool want_meta = o0.key_buf || o0.filter || o0.summary || o0.stats;
-    if (want_meta && (m->max_sstable_bytes != 0 || getenv("B200C_K4_TWO_PASS"))) { c->err = "metadata side band with multi-file output"; return B200C_EUNSUPPORTED; }
+    if (want_meta && getenv("B200C_K4_TWO_PASS")) { c->err = "metadata side band with the two-pass K4 mode (B200C_K4_TWO_PASS)"; return B200C_EUNSUPPORTED; }
     if (want_meta && o0.filter && m->bloom_words && (m->bloom_hash_count <= 0 || m->bloom_words > (1ull << 31))) { c->err = "bloom geometry"; return B200C_EINVAL; }
     if (m->ninputs > MAXK) { c->err = "more than 64 inputs per call"; return B200C_EUNSUPPORTED; }
     if (m->tombstone_option != 0 || m->enforce_strict_liveness) { c->err = "tombstone_option / strict liveness"; return B200C_EUNSUPPORTED; }
@@ -1132,17 +1167,18 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
     uint64_t written_total = 0, samples_total = 0; uint8_t* d_sument = nullptr; uint64_t* d_sumoff = nullptr; uint64_t sument_bound = 0;
     const uint32_t meta_interval = m->min_index_interval > 0 ? (uint32_t)m->min_index_interval : 128u;
     const uint64_t bloom_words = (want_meta && o0.filter) ? m->bloom_words : 0;
+    std::vector<uint8_t> sg_init(want_meta ? sizeof(StatGlobal) : 0, 0);          // initial StatGlobal (a multi-file call resets to it per file)
     if (want_meta) {
         B200C_TRY(ws_typed(c, WS_META_SG, 1, &d_sg));
         B200C_TRY(ws_typed(c, WS_META_TD, 1, &d_td));
         B200C_TRY(ws_typed(c, WS_META_BLOOM, bloom_words * 2 + 16, &d_bloom));
         B200C_TRY(ws_typed(c, WS_META_KEYS, (size_t)2 * 65536, &d_mkeys));
-        std::vector<uint8_t> init(sizeof(StatGlobal), 0); StatGlobal* g0 = (StatGlobal*)init.data();
+        StatGlobal* g0 = (StatGlobal*)sg_init.data();
         g0->min_ts = I64_MAX; g0->max_ts = I64_MIN; g0->min_ldt = I64_MAX; g0->max_ldt = I64_MIN; g0->min_ttl = INT_MAX; g0->max_ttl = INT_MIN;
         auto offsets = [](long long* o, int n) { long long last = 1; o[0] = 1; for (int i = 1; i < n; i++) { long long next = llround((double)last * 1.2); if (next == last) next++; o[i] = next; last = next; } };
         offsets(g0->psize_off, META_PSIZE - 1); offsets(g0->cells_off, META_CELLS - 1);       // EstimatedHistogram.newOffsets (S/utils/EstimatedHistogram.java:91-109)
-        B200C_CUDA_TRY(c, cudaMemcpyAsync(d_sg, init.data(), sizeof(StatGlobal), cudaMemcpyHostToDevice, st));
-        B200C_CUDA_TRY(c, cudaStreamSynchronize(st));                                            // (init is a stack vector)
+        B200C_CUDA_TRY(c, cudaMemcpyAsync(d_sg, sg_init.data(), sizeof(StatGlobal), cudaMemcpyHostToDevice, st));
+        B200C_CUDA_TRY(c, cudaStreamSynchronize(st));                                            // (sg_init is pageable host memory)
         B200C_CUDA_TRY(c, cudaMemsetAsync(d_td, 0, sizeof(TdropTable), st));
         B200C_CUDA_TRY(c, cudaMemsetAsync(d_td->key, 0xFF, sizeof(d_td->key), st));
         if (bloom_words) B200C_CUDA_TRY(c, cudaMemsetAsync(d_bloom, 0, bloom_words * 8, st));
@@ -1493,6 +1529,8 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
     uint8_t *UOUT = nullptr, *IOUT = nullptr, *ISCR = nullptr;
     K4Args ka; memset(&ka, 0, sizeof(ka));
     std::function<int(int)> launch_k4;
+    std::function<int(uint64_t, uint64_t)> launch_k4_stats;
+    uint32_t* d_ccount = nullptr; uint32_t* d_wflag = nullptr; uint64_t* d_wrank = nullptr;     // side band: cells per partition, written flags / ranks
 
     for (int r = 0; r < nr; r++) {
         B200C_TRY(check_cancel());
@@ -1590,12 +1628,11 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
         ka.P = dP; ka.contrib = d_contrib; ka.op_first = d_opfirst; ka.list = d_list; ka.upos = d_upos; ka.pbase = d_pbase; ka.kp = d_kp; ka.klen = d_klen; ka.tok = d_tok;
         ka.dsize = d_dsize; ka.ipay = d_ipay; ka.nblk = d_nblk; ka.ihead = d_ihead; ka.st_munf = d_stmunf; ka.st_rows = d_strows; ka.ovf = d_ovf;
         ka.dpos = d_dpos; ka.ipos = d_ipos; ka.err = d_err; ka.jlo = 0; ka.jhi = nparts; ka.m3_nblk = two_pass ? 1 : 0;
-        uint32_t* d_ccount = nullptr; uint32_t* d_wflag = nullptr; uint64_t* d_wrank = nullptr;
         if (want_meta) {
             B200C_TRY(ws_typed(c, WS_CCOUNT, nparts + 1, &d_ccount));
             B200C_TRY(ws_typed(c, WS_META_FLAG, nparts + 1, &d_wflag));
             B200C_TRY(ws_typed(c, WS_META_WRANK, nparts + 2, &d_wrank));
-            ka.sg = d_sg; ka.td = d_td; ka.ccount = d_ccount;
+            if (!lcs) { ka.sg = d_sg; ka.td = d_td; ka.ccount = d_ccount; }      // multi-file: per file, by k_partition_stats (launch_k4_stats)
         }
         // one launch per fan-in class over its slice of the sorted list
         const uint64_t np_ = nparts;
@@ -1639,6 +1676,33 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
             }
             return B200C_OK;
         };
+        // statistics of the output file holding partitions [jlo, jhi) into d_sg / d_td (multi-file output with the side band)
+        launch_k4_stats = [&, n_le8, n_le12, n_le16, np_, smem8, smem12, smem16, smem64](uint64_t jlo, uint64_t jhi) -> int {
+            K4Args sa = ka; sa.sg = d_sg; sa.td = d_td; sa.ccount = d_ccount; sa.jlo = jlo; sa.jhi = jhi;
+            if (hp.ncx || hp.ctr_mask || hp.sctr_mask) {
+                if (n_le8) B200C_LAUNCH(c, (k_partition_stats<8, 128, true>), (unsigned)((n_le8 + 127) / 128), 128, smem8, sa, 0ull, n_le8);
+                if (n_le12 > n_le8) B200C_LAUNCH(c, (k_partition_stats<12, 64, true>), (unsigned)((n_le12 - n_le8 + 63) / 64), 64, smem12, sa, n_le8, n_le12);
+                if (n_le16 > n_le12) B200C_LAUNCH(c, (k_partition_stats<16, 64, true>), (unsigned)((n_le16 - n_le12 + 63) / 64), 64, smem16, sa, n_le12, n_le16);
+                if (np_ > n_le16) B200C_LAUNCH(c, (k_partition_stats<64, 32, true>), (unsigned)((np_ - n_le16 + 31) / 32), 32, smem64, sa, n_le16, np_);
+            } else {
+                if (n_le8) B200C_LAUNCH(c, (k_partition_stats<8, 128, false>), (unsigned)((n_le8 + 127) / 128), 128, smem8, sa, 0ull, n_le8);
+                if (n_le12 > n_le8) B200C_LAUNCH(c, (k_partition_stats<12, 64, false>), (unsigned)((n_le12 - n_le8 + 63) / 64), 64, smem12, sa, n_le8, n_le12);
+                if (n_le16 > n_le12) B200C_LAUNCH(c, (k_partition_stats<16, 64, false>), (unsigned)((n_le16 - n_le12 + 63) / 64), 64, smem16, sa, n_le12, n_le16);
+                if (np_ > n_le16) B200C_LAUNCH(c, (k_partition_stats<64, 32, false>), (unsigned)((np_ - n_le16 + 31) / 32), 32, smem64, sa, n_le16, np_);
+            }
+            return B200C_OK;
+        };
+        if (want_meta && lcs && c->k4st_attr_set != (int)(smem8 + 1)) {
+            cudaFuncSetAttribute(k_partition_stats<8, 128, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem8);
+            cudaFuncSetAttribute(k_partition_stats<12, 64, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem12);
+            cudaFuncSetAttribute(k_partition_stats<16, 64, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem16);
+            cudaFuncSetAttribute(k_partition_stats<64, 32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem64);
+            cudaFuncSetAttribute(k_partition_stats<8, 128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem8);
+            cudaFuncSetAttribute(k_partition_stats<12, 64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem12);
+            cudaFuncSetAttribute(k_partition_stats<16, 64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem16);
+            cudaFuncSetAttribute(k_partition_stats<64, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem64);
+            c->k4st_attr_set = (int)(smem8 + 1);
+        }
         if (c->k4_attr_set != (int)(smem8 + 1)) {      // > 48 KiB of dynamic shared memory needs an explicit opt-in, once per context/device
             cudaFuncSetAttribute(k_partition_thr<8, 128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem8);
             cudaFuncSetAttribute(k_partition_thr<8, 128, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem8);
@@ -1711,7 +1775,7 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
             B200C_CUDA_TRY(c, cudaMemcpyAsync(h, d_dpos + nparts, 8, cudaMemcpyDeviceToHost, st));
             B200C_CUDA_TRY(c, cudaMemcpyAsync(h + 1, d_ipos + nparts, 8, cudaMemcpyDeviceToHost, st));
             B200C_CUDA_TRY(c, cudaMemcpyAsync(h + 2, d_err, 8, cudaMemcpyDeviceToHost, st));
-            if (want_meta) {
+            if (want_meta && !lcs) {                   // (multi-file: per file, in the writer loop below)
                 B200C_LAUNCH(c, k_written_flags, (unsigned)((nparts + 255) / 256), 256, 0, nparts, d_dsize, d_wflag);
                 B200C_TRY(exclusive_scan<uint32_t>(c, d_wflag, nparts, d_wrank, WS_SCANA, 0));
                 B200C_CUDA_TRY(c, cudaMemcpyAsync(h + 3, d_wrank + nparts, 8, cudaMemcpyDeviceToHost, st));
@@ -1747,7 +1811,7 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
                 B200C_TRY(launch_k4(3));
             }
         }
-        if (want_meta && nparts && ulen_out) {
+        if (want_meta && !lcs && nparts && ulen_out) {
             // per key / per partition metadata of this piece: bloom bits, HLL registers, histograms, index-summary samples, first / last key
             const uint64_t nwritten = h[3];
             const uint64_t ns = (written_total + nwritten + meta_interval - 1) / meta_interval - (written_total + meta_interval - 1) / meta_interval;
@@ -1847,15 +1911,16 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
         B200C_CUDA_TRY(c, cudaMemcpyAsync(g, d_sg, sizeof(StatGlobal), cudaMemcpyDeviceToHost, st));
         B200C_CUDA_TRY(c, cudaStreamSynchronize(st));
         out.first_key_len = written_total ? g->first_len : 0; out.last_key_len = written_total ? g->last_len : 0;
-        if (out.key_buf) {
-            if (out.key_cap < (uint64_t)out.first_key_len + out.last_key_len) { c->err = "key buffer too small"; return B200C_ETOOSMALL; }
+        int mrc = B200C_OK;                                 // a component that does not fit is skipped; the others (and every *_len) are still filled
+        if (out.key_buf && out.key_cap < (uint64_t)out.first_key_len + out.last_key_len) { c->err = "key buffer too small"; mrc = B200C_ETOOSMALL; }
+        else if (out.key_buf) {
             if (out.first_key_len) B200C_CUDA_TRY(c, cudaMemcpyAsync(out.key_buf, d_mkeys, out.first_key_len, cudaMemcpyDeviceToHost, st));
             if (out.last_key_len) B200C_CUDA_TRY(c, cudaMemcpyAsync(out.key_buf + out.first_key_len, d_mkeys + 65536, out.last_key_len, cudaMemcpyDeviceToHost, st));
         }
         if (out.filter) {                                   // BloomFilterSerializer.serialize: i32 hashCount | i32 words | bitset bytes
             out.filter_len = bloom_words ? 8 + bloom_words * 8 : 0;
-            if (out.filter_len > out.filter_cap) { c->err = "filter buffer too small"; return B200C_ETOOSMALL; }
-            if (bloom_words) {
+            if (out.filter_len > out.filter_cap) { c->err = "filter buffer too small"; mrc = B200C_ETOOSMALL; }
+            else if (bloom_words) {
                 const uint32_t k = (uint32_t)m->bloom_hash_count, w = (uint32_t)bloom_words;
                 uint8_t hd[8] = {(uint8_t)(k >> 24), (uint8_t)(k >> 16), (uint8_t)(k >> 8), (uint8_t)k, (uint8_t)(w >> 24), (uint8_t)(w >> 16), (uint8_t)(w >> 8), (uint8_t)w};
                 memcpy(out.filter, hd, 8);
@@ -1865,8 +1930,8 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
         if (out.summary) {                                  // IndexSummarySerializer.serialize + first / last key (S/io/sstable/indexsummary/IndexSummary.java:401-423)
             const uint64_t n = samples_total, eb = sument_bound, fl = out.first_key_len, ll = out.last_key_len;
             out.summary_len = written_total ? 24 + 4 * n + eb + 4 + fl + 4 + ll : 0;
-            if (out.summary_len > out.summary_cap) { c->err = "summary buffer too small"; return B200C_ETOOSMALL; }
-            if (written_total) {
+            if (out.summary_len > out.summary_cap) { c->err = "summary buffer too small"; mrc = B200C_ETOOSMALL; }
+            else if (written_total) {
                 uint8_t* p = out.summary;
                 auto be32 = [&](uint32_t v) { *p++ = (uint8_t)(v >> 24); *p++ = (uint8_t)(v >> 16); *p++ = (uint8_t)(v >> 8); *p++ = (uint8_t)v; };
                 auto be64 = [&](uint64_t v) { be32((uint32_t)(v >> 32)); be32((uint32_t)v); };
@@ -1898,7 +1963,74 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
             for (int i = 0; i < META_HLL; i++) s->hll_registers[i] = (uint8_t)g->hll[i];
         }
         B200C_CUDA_TRY(c, cudaStreamSynchronize(st));
-        return B200C_OK;
+        return mrc;
+    };
+    // side band of one file of a multi-file output: partitions [jlo, jhi), Index.db positions relative to the file (iposf). Every file starts
+    // from a fresh StatGlobal, tombstone table, bloom filter and summary; ranks count from the file's first written partition.
+    // B200C_LCS_META_SPLIT=<file>: append one JSON line per file with where its side band's time goes (tools/bench_lcs_metadata.py)
+    const char* split_path = lcs && want_meta ? getenv("B200C_LCS_META_SPLIT") : nullptr;
+    int split_file = 0;
+    auto file_meta = [&](uint64_t jlo, uint64_t jhi, const uint64_t* iposf, b200c_output& out) -> int {
+        const uint64_t cnt = jhi - jlo;
+        cudaEvent_t sev[4] = {nullptr, nullptr, nullptr, nullptr}; auto sw0 = std::chrono::steady_clock::now(), sw1 = sw0, sw2 = sw0;
+        if (split_path) for (auto& e : sev) cudaEventCreate(&e);
+        if (split_path) cudaEventRecord(sev[0], st);
+        B200C_CUDA_TRY(c, cudaMemcpyAsync(d_sg, sg_init.data(), sizeof(StatGlobal), cudaMemcpyHostToDevice, st));
+        B200C_CUDA_TRY(c, cudaMemsetAsync(d_td, 0, sizeof(TdropTable), st));
+        B200C_CUDA_TRY(c, cudaMemsetAsync(d_td->key, 0xFF, sizeof(d_td->key), st));
+        if (bloom_words) B200C_CUDA_TRY(c, cudaMemsetAsync(d_bloom, 0, bloom_words * 8, st));
+        B200C_TRY(launch_k4_stats(jlo, jhi));
+        if (split_path) cudaEventRecord(sev[1], st);
+        B200C_LAUNCH(c, k_written_flags, (unsigned)((cnt + 255) / 256), 256, 0, cnt, d_dsize + jlo, d_wflag);
+        B200C_TRY(exclusive_scan<uint32_t>(c, d_wflag, cnt, d_wrank, WS_SCANA, 0));
+        B200C_CUDA_TRY(c, cudaMemcpyAsync(h + 3, d_wrank + cnt, 8, cudaMemcpyDeviceToHost, st));
+        B200C_CUDA_TRY(c, cudaMemcpyAsync(h + 5, d_err, 8, cudaMemcpyDeviceToHost, st));
+        B200C_CUDA_TRY(c, cudaStreamSynchronize(st));                  // (also: sg_init has been copied)
+        if ((h[5] >> 56) == 9 || (h[5] >> 56) == 4) {                                         // the statistics pass refused a partition the serialisation pass wrote
+            res->corruption.input = (int)((h[5] >> 48) & 0xFF); res->corruption.kind = 4; res->corruption.chunk = 0; res->corruption.offset = h[5] & 0xFFFFFFFFFFFFull;
+            timing_end(c);
+            c->err = std::string((h[5] >> 56) == 9 ? "unsupported feature" : "malformed Data.db") + " in input " + std::to_string(res->corruption.input) + " (statistics pass of an output file)";
+            return (h[5] >> 56) == 9 ? B200C_EUNSUPPORTED : B200C_ECORRUPT;
+        }
+        if (split_path) sw1 = std::chrono::steady_clock::now();
+        const uint64_t nwritten = h[3], ns = (nwritten + meta_interval - 1) / meta_interval;
+        uint32_t *d_samplej, *d_esize; uint64_t* d_epos;
+        B200C_TRY(ws_typed(c, WS_META_SAMPLE, ns + 1, &d_samplej));
+        B200C_TRY(ws_typed(c, WS_META_ESIZE, ns + 1, &d_esize));
+        B200C_TRY(ws_typed(c, WS_META_EPOS, ns + 2, &d_epos));
+        MetaArgs ma; memset(&ma, 0, sizeof(ma));
+        ma.P = dP; ma.contrib = d_contrib; ma.op_first = d_opfirst + jlo; ma.upos = d_upos; ma.pbase = d_pbase; ma.dsize = d_dsize + jlo; ma.ipos = iposf + jlo; ma.ihead = d_ihead + jlo;
+        ma.ccount = d_ccount + jlo; ma.wrank = d_wrank; ma.nparts = cnt; ma.index_base = 0; ma.written_base = 0; ma.sg = d_sg;
+        ma.bloom = d_bloom; ma.bloom_bits = bloom_words * 64; ma.bloom_k = m->bloom_hash_count; ma.interval = meta_interval; ma.sample_j = d_samplej;
+        ma.first_key = d_mkeys; ma.last_key = d_mkeys + 65536;
+        if (cnt) B200C_LAUNCH(c, k_meta_keys, (unsigned)((cnt + 255) / 256), 256, 0, ma);
+        written_total = nwritten; samples_total = 0; sument_bound = 0;
+        if (ns && o0.summary) {
+            B200C_LAUNCH(c, k_summary_sizes, (unsigned)((ns + 255) / 256), 256, 0, ma, ns, d_esize);
+            B200C_TRY(exclusive_scan<uint32_t>(c, d_esize, ns, d_epos, WS_SCANA, 0));
+            B200C_CUDA_TRY(c, cudaMemcpyAsync(h + 4, d_epos + ns, 8, cudaMemcpyDeviceToHost, st));
+            B200C_CUDA_TRY(c, cudaStreamSynchronize(st));
+            B200C_TRY(ws_typed(c, WS_META_SUMENT, h[4] + 64, &d_sument));
+            B200C_TRY(ws_typed(c, WS_META_SUMOFF, ns + 2, &d_sumoff));
+            B200C_LAUNCH(c, k_summary_emit, (unsigned)((ns + 255) / 256), 256, 0, ma, ns, d_epos, d_sument, d_sumoff);
+            sument_bound = h[4]; samples_total = ns;
+        }
+        if (split_path) { cudaEventRecord(sev[2], st); B200C_CUDA_TRY(c, cudaStreamSynchronize(st)); sw2 = std::chrono::steady_clock::now(); }
+        const int mrc = finish_meta(out);
+        if (split_path) {
+            cudaEventRecord(sev[3], st); cudaEventSynchronize(sev[3]);
+            const auto sw3 = std::chrono::steady_clock::now();
+            float ms[3] = {0, 0, 0}; for (int k = 0; k < 3; k++) cudaEventElapsedTime(&ms[k], sev[k], sev[k + 1]);
+            auto wall = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
+            if (FILE* fp = fopen(split_path, "a")) {
+                fprintf(fp, "{\"file\": %d, \"partitions\": %llu, \"stats_pass_ms\": %.3f, \"keys_summary_ms\": %.3f, \"finish_ms\": %.3f, \"wall_stats_ms\": %.3f, \"wall_keys_summary_ms\": %.3f, \"wall_finish_ms\": %.3f}\n",
+                        split_file, (unsigned long long)cnt, ms[0], ms[1], ms[2], wall(sw0, sw1), wall(sw1, sw2), wall(sw2, sw3));
+                fclose(fp);
+            }
+            for (auto& e : sev) cudaEventDestroy(e);
+            split_file++;
+        }
+        return mrc;
     };
     if (to_host_stream) {
         b200c_output& out = out0;
@@ -1966,7 +2098,7 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
         while (jlo < nparts && start_b < ulen_out) {
             B200C_TRY(check_cancel());
             const uint64_t remaining = ulen_out - start_b, rem_chunks = (remaining + L - 1) / L;
-            uint64_t want = std::max<uint64_t>(64, (uint64_t)((double)m->max_sstable_bytes / est_ratio * 1.08) / L + 8), done = 0, jhi = nparts, status = 2;
+            uint64_t want = std::max<uint64_t>(64, (uint64_t)std::min(1e18, (double)m->max_sstable_bytes / est_ratio * 1.08) / L + 8), done = 0, jhi = nparts, status = 2;
             while (status == 2) {
                 uint64_t W = std::min(rem_chunks, want);
                 if (W > done) B200C_TRY(compress_slots_device(c, comp, UOUT + start_b + done * L, std::min(remaining - done * L, (W - done) * (uint64_t)L), (int)L,
@@ -2024,6 +2156,7 @@ int b200c_compact(b200c_ctx* c, const b200c_manifest* m, b200c_result* res, int 
                         o.data_len = out_len; o.index_len = filen; o.nchunks = fchunks; o.data_length = flen; o.digest = digest;
                         o.partitions = fs.partitions_out; o.rows = fs.rows_out;
                     }
+                    if (want_meta) { const int mrc = file_meta(jlo, jhi, d_iposf, o); if (mrc == B200C_ETOOSMALL) rc = mrc; else B200C_TRY(mrc); }
                 }
                 f++;
             }

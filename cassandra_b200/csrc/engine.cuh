@@ -36,7 +36,7 @@ struct b200c_ctx {
     cudaEvent_t ev_stage[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     double stage_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     int nstages = 0;
-    int k4_attr_set = 0, k4s_attr_set = 0;
+    int k4_attr_set = 0, k4s_attr_set = 0, k4st_attr_set = 0;
     cudaStream_t copy_stream = nullptr;            // host->device staging of the inputs, overlapped with K1 input by input
     cudaEvent_t ev_in[64] = {};
     std::vector<cudaEvent_t> ev_marks;             // timed events of the stage clock (grown on demand)

@@ -216,7 +216,9 @@ typedef struct b200c_manifest {
     /* token range (lo, hi] handled by this call; lo = INT64_MIN and hi = INT64_MAX for the whole ring */
     int64_t         token_lo;
     int64_t         token_hi;
-    /* LCS: switch output file when on-disk bytes exceed this (MaxSSTableSizeWriter.java:76-79); 0 = single output */
+    /* LCS: switch output file when on-disk bytes exceed this (MaxSSTableSizeWriter.java:76-79); 0 = single output. A multi-file call
+       returns one b200c_output per file, each with its own side band (Filter.db, Summary.db, first / last key, b200c_sstable_stats) as
+       that file's writer would have gathered it; INT64_MAX (a level-0 user-defined LCS task) = one file through the same path */
     uint64_t        max_sstable_bytes;
     int32_t         partitioner;        /* B200C_PARTITIONER_* */
     /* optional purge table (CompactionController.getPurgeEvaluator is per partition key, S/db/compaction/CompactionController.java:
@@ -227,7 +229,9 @@ typedef struct b200c_manifest {
     const int64_t*  purge_range_hi;
     const int64_t*  purge_range_max_ts;
     /* Filter.db geometry, decided by the host as FilterFactory.getFilter(estimatedKeys, fpChance) does (S/utils/FilterFactory.java:
-       60-75, BloomCalculations): K hash functions over bloom_words 64-bit words, per output file. 0 words = no filter (fpChance 1.0). */
+       60-75, BloomCalculations): K hash functions over bloom_words 64-bit words, per output file. 0 words = no filter (fpChance 1.0).
+       The same geometry applies to every file of a multi-file call: MaxSSTableSizeWriter sizes each writer's filter for
+       sstableKeyCount() = estimatedTotalKeys / estimatedSSTables, the same for all of them (CompactionAwareWriter.java:230-250). */
     int32_t         bloom_hash_count;
     int32_t         min_index_interval; /* Summary.db sampling (128 default, S/schema/TableParams.java); 0 = 128 */
     uint64_t        bloom_words;
@@ -265,7 +269,7 @@ typedef struct b200c_sstable_stats {
     uint8_t  hll_registers[1 << B200C_HLL_P];
 } b200c_sstable_stats;
 
-typedef struct b200c_output {           /* one output sstable; caller provides the buffers */
+typedef struct b200c_output {           /* one output sstable (one per file of a multi-file call, each with its own side band); caller provides the buffers */
     uint8_t*  data;        uint64_t data_cap;     uint64_t data_len;      /* Data.db image */
     uint8_t*  index;       uint64_t index_cap;    uint64_t index_len;     /* Index.db image */
     uint64_t* chunk_offsets; uint64_t chunk_cap;  uint64_t nchunks;       /* CompressionInfo.db chunk offsets */
@@ -274,7 +278,10 @@ typedef struct b200c_output {           /* one output sstable; caller provides t
     uint32_t  _pad;
     uint64_t  partitions;                                                 /* partitions written */
     uint64_t  rows;                                                       /* rows + markers written */
-    /* ---- the rest of the sstable (SURVEY §8 f1), all optional: a NULL pointer skips that component. HOST pointers always. ---- */
+    /* ---- the rest of the sstable (SURVEY §8 f1), all optional: a NULL pointer skips that component. HOST pointers always.
+       outputs[0] decides which components the call computes; in a multi-file call every slot gets its file's own. Capacities are
+       checked per slot: a slot too small for its key / filter / summary makes the call return B200C_ETOOSMALL with the lengths that
+       slot needs in *_len. Refused (B200C_EUNSUPPORTED) under the two-pass K4 A/B mode (B200C_K4_TWO_PASS). ---- */
     /* first / last partition key written (SortedTableWriter.endPartition :247-250; StatsMetadata.firstKey/lastKey, Summary.db tail):
        key_buf receives first key then last key back to back; lengths below. Needs key_cap >= first_key_len + last_key_len
        (2 * 65535 always suffices). */

@@ -24,6 +24,9 @@ import java.util.Map;
 import java.util.Set;
 
 import org.apache.cassandra.config.DatabaseDescriptor;
+import org.apache.cassandra.db.Directories;
+import org.apache.cassandra.db.compaction.writers.CompactionAwareWriter;
+import org.apache.cassandra.db.compaction.writers.MaxSSTableSizeWriter;
 import org.apache.cassandra.db.ColumnFamilyStore;
 import org.apache.cassandra.db.SerializationHeader;
 import org.apache.cassandra.db.Slice;
@@ -66,9 +69,42 @@ import static org.apache.cassandra.db.compaction.B200C.Layout.*;
 
 public class GpuCompactionTask extends CompactionTask
 {
+    private final int level;                 // level of the output sstables (Statistics.db sstableLevel)
+    private final long maxSSTableBytes;      // 0: one output (DefaultCompactionWriter); else MaxSSTableSizeWriter's switch limit, Long.MAX_VALUE included
+
     public GpuCompactionTask(ColumnFamilyStore cfs, LifecycleTransaction txn, long gcBefore)
     {
+        this(cfs, txn, gcBefore, 0, 0L);
+    }
+
+    /** a leveled task (LeveledCompactionTask without majorCompaction): outputs of at most maxSSTableBytes on disk, written at `level` */
+    public GpuCompactionTask(ColumnFamilyStore cfs, LifecycleTransaction txn, long gcBefore, int level, long maxSSTableBytes)
+    {
         super(cfs, txn, gcBefore);
+        this.level = level;
+        this.maxSSTableBytes = maxSSTableBytes;
+    }
+
+    @Override
+    protected int getLevel()
+    {
+        return level;
+    }
+
+    /** the writer of the stock path (super.runMayThrow() after B200C_EUNSUPPORTED): a leveled task keeps LeveledCompactionTask's
+     *  MaxSSTableSizeWriter (LeveledCompactionTask.java:46-54), so the fallback writes files of maxSSTableBytes at the task's level too */
+    @Override
+    public CompactionAwareWriter getCompactionAwareWriter(ColumnFamilyStore cfs, Directories directories, LifecycleTransaction txn, Set<SSTableReader> nonExpiredSSTables)
+    {
+        if (maxSSTableBytes > 0)
+            return new MaxSSTableSizeWriter(cfs, directories, txn, nonExpiredSSTables, maxSSTableBytes, level, false);
+        return super.getCompactionAwareWriter(cfs, directories, txn, nonExpiredSSTables);
+    }
+
+    @Override
+    protected boolean partialCompactionsAcceptable()
+    {
+        return maxSSTableBytes > 0 ? level == 0 : super.partialCompactionsAcceptable();     // LeveledCompactionTask.partialCompactionsAcceptable
     }
 
     // ---- the envelope of include/b200c.h, checked BEFORE a task is built so that unsupported tables keep the stock task -------------------
@@ -236,7 +272,7 @@ public class GpuCompactionTask extends CompactionTask
                 for (SSTableReader r : actuallyCompact) inputs.add(new Input(r));
                 // ---- manifest --------------------------------------------------------------------------------------------------------------
                 ByteBuffer in = B200C.struct(SIZEOF_INPUT * inputs.size());
-                long totalIn = 0, totalIndex = 0;
+                long totalIn = 0, totalIndex = 0, totalCompressed = 0;
                 for (int i = 0; i < inputs.size(); i++)
                 {
                     Input s = inputs.get(i); int o = i * SIZEOF_INPUT;
@@ -259,7 +295,7 @@ public class GpuCompactionTask extends CompactionTask
                     in.putLong(o + IN_HEADER_STATS, hs.minTimestamp).putLong(o + IN_HEADER_STATS + 8, hs.minLocalDeletionTime).putInt(o + IN_HEADER_STATS + 16, hs.minTTL);
                     in.putInt(o + IN_LEVEL, s.reader.getSSTableLevel());
                     in.putLong(o + IN_SUMMARY_POSITIONS, B200C.address(s.summaryPositions)).putLong(o + IN_NSUMMARY, s.nSummary);
-                    totalIn += cm.dataLength; totalIndex += s.index.capacity();
+                    totalIn += cm.dataLength; totalIndex += s.index.capacity(); totalCompressed += s.data.capacity();
                 }
                 CompressionParams cp = table.params.compression;
                 int outComp = compressorId(cp.getSstableCompressor().getClass().getSimpleName());
@@ -288,101 +324,177 @@ public class GpuCompactionTask extends CompactionTask
                 for (org.apache.cassandra.db.memtable.Memtable mt : cfs.getTracker().getView().getAllMemtables()) purgeMax = Math.min(purgeMax, mt.getMinTimestamp());
                 m.putLong(M_PURGE_MAX_TIMESTAMP, controller.compactingRepaired() ? purgeMax : Long.MIN_VALUE);   // only_purge_repaired_tombstones: nothing purgeable
                 m.putLong(M_TOKEN_LO, Long.MIN_VALUE).putLong(M_TOKEN_HI, Long.MAX_VALUE);
-                m.putLong(M_MAX_SSTABLE_BYTES, 0L);                 // STCS: DefaultCompactionWriter, one output
+                m.putLong(M_MAX_SSTABLE_BYTES, maxSSTableBytes);    // 0: DefaultCompactionWriter (STCS); LCS: MaxSSTableSizeWriter, one output per file
                 m.putInt(M_PARTITIONER, table.partitioner instanceof Murmur3Partitioner ? B200C.PARTITIONER_MURMUR3 : B200C.PARTITIONER_BYTE_ORDERED);
                 // Filter.db geometry as SortedTableWriter would choose it (FilterFactory.getFilter(estimatedKeys, fpChance))
                 long estimatedKeys = Math.max(1, SSTableReader.getApproximateKeyCount(actuallyCompact));
+                if (maxSSTableBytes > 0)                            // MaxSSTableSizeWriter: every file's filter is sized for keysPerSSTable (CompactionAwareWriter.sstableKeyCount)
+                    estimatedKeys = Math.max(1, estimatedKeys / Math.max(1, expectedWriteSize(actuallyCompact, estimatedKeys) / maxSSTableBytes));
                 double fp = table.params.bloomFilterFpChance;
                 int[] spec = BloomSpec.of(estimatedKeys, fp);
                 m.putInt(M_BLOOM_HASH_COUNT, spec[0]).putLong(M_BLOOM_WORDS, fp >= 1.0 ? 0L : ((estimatedKeys * spec[1] + 20 - 1) >>> 6) + 1);
                 m.putInt(M_MIN_INDEX_INTERVAL, table.params.minIndexInterval);
 
                 // ---- result + caller-provided output buffers ------------------------------------------------------------------------------------
-                long dataCap = B200C.compressBound(outComp, totalIn, cp.chunkLength());
-                ByteBuffer outData = ByteBuffer.allocateDirect(Math.toIntExact(Math.min(dataCap, Integer.MAX_VALUE - 8)));   // > 2 GiB outputs: use several buffers / Unsafe
-                ByteBuffer outIndex = ByteBuffer.allocateDirect(Math.toIntExact(totalIndex + (1 << 20)));
-                ByteBuffer outOffsets = B200C.struct(Math.toIntExact(8 * (totalIn / cp.chunkLength() + 16)));
-                ByteBuffer keys = ByteBuffer.allocateDirect(2 * 65535);
-                ByteBuffer filter = B200C.struct(Math.toIntExact(8 + 8 * m.getLong(M_BLOOM_WORDS)));
-                ByteBuffer summary = ByteBuffer.allocateDirect(Math.toIntExact(totalIndex / 16 + (1 << 20)));
-                ByteBuffer stats = B200C.struct(SIZEOF_STATS);
-                ByteBuffer out = B200C.struct(SIZEOF_OUTPUT);
-                out.putLong(O_DATA, B200C.address(outData)).putLong(O_DATA_CAP, outData.capacity());
-                out.putLong(O_INDEX, B200C.address(outIndex)).putLong(O_INDEX_CAP, outIndex.capacity());
-                out.putLong(O_CHUNK_OFFSETS, B200C.address(outOffsets)).putLong(O_CHUNK_CAP, outOffsets.capacity() / 8);
-                out.putLong(O_KEY_BUF, B200C.address(keys)).putLong(O_KEY_CAP, keys.capacity());
-                out.putLong(O_FILTER, B200C.address(filter)).putLong(O_FILTER_CAP, filter.capacity());
-                out.putLong(O_SUMMARY, B200C.address(summary)).putLong(O_SUMMARY_CAP, summary.capacity());
-                out.putLong(O_STATS, B200C.address(stats));
-                ByteBuffer res = B200C.struct(SIZEOF_RESULT);
-                res.putInt(R_NOUTPUTS_CAP, 1).putLong(R_OUTPUTS, B200C.address(out));
-                B200C.hostRegister(B200C.address(outData), outData.capacity());
-
-                // ---- the call; progress and stop requests travel through poll / cancel from the CompactionInfo.Holder ------------------------------
-                GpuCompactionInfo info = new GpuCompactionInfo(this, ctx, totalIn);
-                CompactionManager.instance.active.beginCompaction(info);
-                int rc;
-                try
+                // one output slot per file: a single-output task gets buffers for the whole stream; a leveled one starts from the file limit and,
+                // on B200C_ETOOSMALL, calls again with the number of files and the sizes the engine reported (required_*_cap, *_len of each slot)
+                long dataCap = B200C.compressBound(outComp, totalIn, cp.chunkLength()), indexCap = totalIndex + (1 << 20), chunkCap = totalIn / cp.chunkLength() + 16;
+                long summaryCap = totalIndex / 16 + (1 << 20);
+                int nout = 1;
+                if (maxSSTableBytes > 0 && maxSSTableBytes < dataCap)
                 {
-                    if (!cfs.getCompactionStrategyManager().isActive())
-                        throw new CompactionInterruptedException(info.getCompactionInfo());
-                    rc = B200C.compact(ctx, B200C.address(m), B200C.address(res), 0);
+                    // the limit counts ON-DISK (compressed) bytes: the files are about the compressed input over the limit; a file holds the limit plus
+                    // the partition that crosses it (a larger one comes back as ETOOSMALL with its size, and the retry below grows the slots)
+                    long files = Math.max(1, totalCompressed / Math.max(1, maxSSTableBytes) + 2);
+                    nout = (int) Math.min(4096, files);
+                    dataCap = Math.min(dataCap, maxSSTableBytes + (16 << 20)); indexCap = Math.min(indexCap, indexCap / files * 2 + (1 << 20));
+                    chunkCap = Math.min(chunkCap, 4 * dataCap / cp.chunkLength() + 16); summaryCap = Math.min(summaryCap, indexCap / 16 + (1 << 20));
                 }
-                finally
+                Outputs outs = null;
+                ByteBuffer res = B200C.struct(SIZEOF_RESULT);
+                int rc;
+                for (int attempt = 0; ; attempt++)
                 {
-                    CompactionManager.instance.active.finishCompaction(info);
-                    B200C.hostUnregister(B200C.address(outData));
+                    if (outs != null) outs.close();
+                    outs = new Outputs(nout, dataCap, indexCap, chunkCap, summaryCap, 8 + 8 * m.getLong(M_BLOOM_WORDS));
+                    res.putInt(R_NOUTPUTS_CAP, nout).putLong(R_OUTPUTS, B200C.address(outs.slots));
+
+                    // ---- the call; progress and stop requests travel through poll / cancel from the CompactionInfo.Holder ------------------------------
+                    GpuCompactionInfo info = new GpuCompactionInfo(this, ctx, totalIn);
+                    CompactionManager.instance.active.beginCompaction(info);
+                    try
+                    {
+                        if (!cfs.getCompactionStrategyManager().isActive())
+                            throw new CompactionInterruptedException(info.getCompactionInfo());
+                        rc = B200C.compact(ctx, B200C.address(m), B200C.address(res), 0);
+                    }
+                    finally
+                    {
+                        CompactionManager.instance.active.finishCompaction(info);
+                        outs.unregister();
+                    }
+                    if (rc != B200C.ETOOSMALL || attempt == 2) break;
+                    nout = Math.max(nout, res.getInt(R_NOUTPUTS));
+                    dataCap = Math.max(dataCap, res.getLong(R_REQUIRED_DATA_CAP)); indexCap = Math.max(indexCap, res.getLong(R_REQUIRED_INDEX_CAP));
+                    chunkCap = Math.max(chunkCap, res.getLong(R_REQUIRED_CHUNK_CAP));
+                    for (int k = 0; k < Math.min(nout, outs.n); k++) summaryCap = Math.max(summaryCap, outs.slot(k).getLong(O_SUMMARY_LEN));
                 }
                 switch (rc)
                 {
                     case B200C.OK: break;
                     case B200C.ECORRUPT:
                     {
+                        outs.close();
                         SSTableReader bad = inputs.get(res.getInt(R_CORRUPTION)).reader;         // corruption.input
                         bad.markSuspect();
                         throw new CorruptSSTableException(new IOException(B200C.lastError(ctx)), bad.getFilename());
                     }
-                    case B200C.ECANCELLED: throw new CompactionInterruptedException(info.getCompactionInfo());
-                    case B200C.EUNSUPPORTED: super.runMayThrow(); return;                        // an input used a feature outside the envelope: the stock task does it
-                    default: throw new RuntimeException("b200c_compact failed (" + rc + "): " + B200C.lastError(ctx));
+                    case B200C.ECANCELLED: outs.close(); throw new CompactionInterruptedException(new GpuCompactionInfo(this, ctx, totalIn).getCompactionInfo());
+                    case B200C.EUNSUPPORTED: outs.close(); super.runMayThrow(); return;          // an input used a feature outside the envelope: the stock task does it
+                    default: outs.close(); throw new RuntimeException("b200c_compact failed (" + rc + "): " + B200C.lastError(ctx));
                 }
 
-                // ---- outputs -> component files of a new descriptor, tracked by the transaction exactly like a writer's would be ----------------------
-                if (out.getLong(O_PARTITIONS) > 0)
+                // ---- outputs -> component files of a new descriptor each, tracked by the transaction exactly like a writer's would be -----------------
+                long written = 0;
+                for (int k = 0; k < res.getInt(R_NOUTPUTS); k++)
                 {
+                    ByteBuffer out = outs.slot(k);
+                    if (out.getLong(O_PARTITIONS) == 0) continue;
                     Descriptor d = cfs.newSSTableDescriptor(getDirectories().getWriteableLocationAsFile(cfs, null, out.getLong(O_DATA_LEN)));
                     Set<Component> components = new java.util.HashSet<>(d.getFormat().allComponents());
                     transaction.trackNew(new org.apache.cassandra.io.sstable.SSTable.Builder<>(d).setComponents(components).setTableMetadataRef(cfs.metadata).build(cfs));
-                    write(d.fileFor(Components.DATA), outData, out.getLong(O_DATA_LEN));
-                    write(d.fileFor(BigFormat.Components.PRIMARY_INDEX), outIndex, out.getLong(O_INDEX_LEN));
-                    write(d.fileFor(Components.FILTER), filter, out.getLong(O_FILTER_LEN));
-                    write(d.fileFor(BigFormat.Components.SUMMARY), summary, out.getLong(O_SUMMARY_LEN));
-                    writeCompressionInfo(d, cp, out, outOffsets);
+                    write(d.fileFor(Components.DATA), outs.data[k], out.getLong(O_DATA_LEN));
+                    write(d.fileFor(BigFormat.Components.PRIMARY_INDEX), outs.index[k], out.getLong(O_INDEX_LEN));
+                    write(d.fileFor(Components.FILTER), outs.filter[k], out.getLong(O_FILTER_LEN));
+                    write(d.fileFor(BigFormat.Components.SUMMARY), outs.summary[k], out.getLong(O_SUMMARY_LEN));
+                    writeCompressionInfo(d, cp, out, outs.offsets[k]);
                     try (FileOutputStreamPlus o = new FileOutputStreamPlus(d.fileFor(Components.DIGEST)))
                     {
                         o.write(Long.toString(out.getInt(O_DIGEST) & 0xFFFFFFFFL).getBytes(java.nio.charset.StandardCharsets.UTF_8));
                     }
-                    writeStatistics(d, table, header, stats, keys, out, (double) out.getLong(O_DATA_LEN) / Math.max(1, out.getLong(O_DATA_LENGTH)), actuallyCompact, fp);
+                    writeStatistics(d, table, header, outs.stats[k], outs.keys[k], out, (double) out.getLong(O_DATA_LEN) / Math.max(1, out.getLong(O_DATA_LENGTH)), actuallyCompact, fp);
                     d.getFormat().getWriterFactory();                                            // TOC.txt
                     org.apache.cassandra.io.sstable.format.TOCComponent.appendTOC(d, components);
                     SSTableReader reader = SSTableReader.open(cfs, d, components, cfs.metadata);
                     transaction.update(reader, false);
+                    written += out.getLong(O_DATA_LEN);
                 }
+                outs.close();
                 transaction.obsoleteOriginals();
                 transaction.prepareToCommit();
                 transaction.commit();
 
                 long[] merged = new long[inputs.size()];
                 for (int i = 0; i < merged.length; i++) merged[i] = res.getLong(R_MERGED_ROW_COUNTS + 8 * i);
-                updateCompactionHistory(transaction.opId(), cfs.getKeyspaceName(), cfs.getTableName(), merged, totalIn, out.getLong(O_DATA_LEN),
+                updateCompactionHistory(transaction.opId(), cfs.getKeyspaceName(), cfs.getTableName(), merged, totalIn, written,
                                         com.google.common.collect.ImmutableMap.of(COMPACTION_TYPE_PROPERTY, compactionType.type));
-                cfs.metric.compactionBytesWritten.inc(out.getLong(O_DATA_LEN));
+                cfs.metric.compactionBytesWritten.inc(written);
             }
             finally
             {
                 for (Input s : inputs) s.close();
             }
         }
+    }
+
+    /** MaxSSTableSizeWriter.getTotalWriteSize: the expected output size, scaled by the estimated key count after compaction */
+    private long expectedWriteSize(Collection<SSTableReader> sstables, long estimatedTotalKeys)
+    {
+        long before = 0;
+        for (SSTableReader r : sstables) before += r.estimatedKeys();
+        return Math.round((double) estimatedTotalKeys / Math.max(1, before) * cfs.getExpectedCompactedFileSize(sstables, compactionType));
+    }
+
+    /** caller-provided buffers of n output slots (b200c_output), pinned while the call runs */
+    private static final class Outputs implements AutoCloseable
+    {
+        final int n;
+        final ByteBuffer slots;
+        final ByteBuffer[] data, index, offsets, keys, filter, summary, stats;
+
+        Outputs(int n, long dataCap, long indexCap, long chunkCap, long summaryCap, long filterCap)
+        {
+            this.n = n;
+            slots = B200C.struct(SIZEOF_OUTPUT * n);
+            data = new ByteBuffer[n]; index = new ByteBuffer[n]; offsets = new ByteBuffer[n]; keys = new ByteBuffer[n];
+            filter = new ByteBuffer[n]; summary = new ByteBuffer[n]; stats = new ByteBuffer[n];
+            for (int k = 0; k < n; k++)
+            {
+                data[k] = ByteBuffer.allocateDirect(Math.toIntExact(Math.min(dataCap, Integer.MAX_VALUE - 8)));      // > 2 GiB outputs: use several buffers / Unsafe
+                index[k] = ByteBuffer.allocateDirect(Math.toIntExact(indexCap));
+                offsets[k] = B200C.struct(Math.toIntExact(8 * chunkCap));
+                keys[k] = ByteBuffer.allocateDirect(2 * 65535);
+                filter[k] = B200C.struct(Math.toIntExact(filterCap));
+                summary[k] = ByteBuffer.allocateDirect(Math.toIntExact(summaryCap));
+                stats[k] = B200C.struct(SIZEOF_STATS);
+                ByteBuffer o = slot(k);
+                o.putLong(O_DATA, B200C.address(data[k])).putLong(O_DATA_CAP, data[k].capacity());
+                o.putLong(O_INDEX, B200C.address(index[k])).putLong(O_INDEX_CAP, index[k].capacity());
+                o.putLong(O_CHUNK_OFFSETS, B200C.address(offsets[k])).putLong(O_CHUNK_CAP, offsets[k].capacity() / 8);
+                o.putLong(O_KEY_BUF, B200C.address(keys[k])).putLong(O_KEY_CAP, keys[k].capacity());
+                o.putLong(O_FILTER, B200C.address(filter[k])).putLong(O_FILTER_CAP, filter[k].capacity());
+                o.putLong(O_SUMMARY, B200C.address(summary[k])).putLong(O_SUMMARY_CAP, summary[k].capacity());
+                o.putLong(O_STATS, B200C.address(stats[k]));
+                B200C.hostRegister(B200C.address(data[k]), data[k].capacity());
+            }
+        }
+
+        /** view of slot k (native order, offsets from B200C.Layout) */
+        ByteBuffer slot(int k)
+        {
+            ByteBuffer b = slots.duplicate().order(slots.order()); b.position(k * SIZEOF_OUTPUT).limit((k + 1) * SIZEOF_OUTPUT);
+            return b.slice().order(slots.order());
+        }
+
+        private boolean registered = true;
+        void unregister()
+        {
+            if (!registered) return;
+            for (ByteBuffer b : data) B200C.hostUnregister(B200C.address(b));
+            registered = false;
+        }
+
+        public void close() { unregister(); }
     }
 
     private static void write(File f, ByteBuffer b, long n) throws IOException
@@ -432,7 +544,7 @@ public class GpuCompactionTask extends CompactionTask
         components.put(MetadataType.VALIDATION, new ValidationMetadata(table.partitioner.getClass().getCanonicalName(), fpChance));
         components.put(MetadataType.STATS, new StatsMetadata(new EstimatedHistogram(psizeOffsets, psize), new EstimatedHistogram(cellOffsets, cells), intervals.build(),
                                                              s.getLong(S_MIN_TIMESTAMP), s.getLong(S_MAX_TIMESTAMP), s.getLong(S_MIN_LDT), s.getLong(S_MAX_LDT),
-                                                             s.getInt(S_MIN_TTL), s.getInt(S_MAX_TTL), ratio, th.build(), getLevel(), table.comparator.subtypes(), Slice.ALL,
+                                                             s.getInt(S_MIN_TTL), s.getInt(S_MAX_TTL), ratio, th.build(), level, table.comparator.subtypes(), Slice.ALL,
                                                              s.getInt(S_HAS_LEGACY_COUNTER_SHARDS) != 0, ActiveRepairService.UNREPAIRED_SSTABLE, s.getLong(S_TOTAL_COLUMNS_SET), s.getLong(S_TOTAL_ROWS), Double.NaN,
                                                              org.apache.cassandra.service.StorageService.instance.getLocalHostUUID(), null, false,
                                                              s.getInt(S_HAS_PARTITION_DELETIONS) != 0, ByteBuffer.wrap(first), ByteBuffer.wrap(last)));
